@@ -134,6 +134,16 @@ def synth_batch(B: int, seed: int):
     return wave, ids
 
 
+def dump_outputs(out_dir, generated_ids):
+    """Writes what the timed path returned in its last step -- the generated ids [global batch, prompt + new tokens], prompt
+    included, as generate() returns them -- to out_dir/generated_ids.npy.  Inputs and weights are seeded, so two builds run with
+    the same arguments can be compared output for output.  The ids are stored as float64, a floating-point format in which they
+    are exact."""
+    d = Path(out_dir)
+    d.mkdir(parents=True, exist_ok=True)
+    np.save(d / "generated_ids.npy", generated_ids.cpu().numpy().astype(np.float64))
+
+
 def init_synthetic_weights_(model, seed: int):
     """Random-init weights of the AF3-7B architecture directly on the GPU (no checkpoint exists offline):
     N(0, 0.02) matrices / embeddings, zero biases, unit norm gains -- the reference's default init family."""
@@ -294,6 +304,7 @@ def run_ours(args):
         barrier()
         ops.LAUNCHES = 0
         stages = []
+        out = None
         e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         e0.record()
         for _ in range(n_steps):
@@ -303,7 +314,7 @@ def run_ours(args):
                 ev.record()
                 model.stage_events.append(("step_start", ev))
                 model.stage_host_t = []
-            step(from_host)
+            out = step(from_host)
             if collect_stages:
                 stages.append(model.stage_events)
                 host_t.append(model.stage_host_t)
@@ -318,7 +329,7 @@ def run_ours(args):
             t = torch.tensor([ms], device=dev)
             dist.all_reduce(t, op=dist.ReduceOp.MAX)
             ms = float(t.item())
-        return ms, ops.LAUNCHES, stages
+        return ms, ops.LAUNCHES, stages, out
 
     # The clock sampler (one long-lived `nvidia-smi -lms` process) is started BEFORE the warm-up steps: its start-up (NVML attach)
     # stalls work submission on the GPU for a while, which must not land inside the timed region.  AF3_BENCH_SAMPLER=late
@@ -334,14 +345,16 @@ def run_ours(args):
     if rank == 0 and sampler_mode == "late":
         sampler.start()
     thr0 = cpu_throttle_snapshot()
-    ms_dev, launches, stages = timed(args.steps, from_host=False, collect_stages=True)
+    ms_dev, launches, stages, last_out = timed(args.steps, from_host=False, collect_stages=True)
     thr1 = cpu_throttle_snapshot()
     host_cpu = {"cpus_allowed": len(os.sched_getaffinity(0)), "loadavg": os.getloadavg()[0],
                 "throttled_during_timed": None if (thr0 is None or thr1 is None) else
                 {"nr": thr1["nr_throttled"] - thr0["nr_throttled"], "ms": round(thr1["throttled_ms"] - thr0["throttled_ms"], 1)}}
     clocks = sampler.stop() if (rank == 0 and sampler_mode != "off") else None
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, last_out)
     step(True)  # warm the host path (pinned staging, H2D)
-    ms_e2e, _, _ = timed(args.steps, from_host=True)
+    ms_e2e, _, _, _ = timed(args.steps, from_host=True)
 
     # one profiled step (per-kernel CUDA events around every launch; PDL off so kernels do not overlap their brackets;
     # the decode steps replayed from the CUDA graph are not bracketed, the first -- eager -- decode step is)
@@ -793,17 +806,9 @@ def run_reference(args):
     if rank != 0:
         return
     ref = CpuReference(layers=4, n_win=1, n_dec=2)
-    t0 = time.time()
-    for _ in range(max(args.warmup, 0)):
+    for _ in range(args.warmup):
         ref.sample()
-        if time.time() - t0 > 60:
-            break
-    vals = []
-    t0 = time.time()
-    for _ in range(max(args.steps, 1)):
-        vals.append(ref.sample())
-        if time.time() - t0 > 150:  # keep the whole run within a few minutes on small hosts
-            break
+    vals = [ref.sample() for _ in range(args.steps)]
     total = sum(r["estimated_workload_seconds"] for r in vals) / len(vals)
     v = B_PER_GPU * NEW_TOKENS / total
     res = dict(vals[-1], value=v)
@@ -830,7 +835,15 @@ def main():
     ap.add_argument("--no-extras", action="store_true", help="skip the BASELINE config 3 / config 5 / 256-window log-mel measurements")
     ap.add_argument("--scaling", default="weak", choices=["weak", "strong"],
                     help="weak (driver contract): 32 clips per GPU; strong: a global batch of 32 split over the ranks")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write the generated ids of the last timed step to DIR/generated_ids.npy (float64)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.warmup < 0:
+        ap.error("--warmup must not be negative")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs applies to --impl ours (the reference arm times CPU samples, it returns no ids)")
     if args.impl == "reference":
         run_reference(args)
         return
